@@ -1,7 +1,11 @@
 """bench.py -- optimizer steps/s of the DotaClient optimizer hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c1]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c1] [--dump-outputs DIR]
     torchrun --nproc-per-node N bench.py --gpus N ...        (one rank per GPU, NCCL)
+
+``--dump-outputs DIR`` writes what the last timed train() step handed its caller (rank 0) as DIR/<name>.npy: the loss
+terms, per-head entropies and grad norms it returns, and the policy parameters it updated (see ``step_outputs``).  Inputs
+and initial weights are seeded, so two builds run with the same arguments can be compared output for output.
 
 A "step" is one ``DotaOptimizer.train()`` call (forward, PPO loss, backward, gradient all-reduce, clip, Adam)
 on one synthetic experience batch.  Default workload = BASELINE.json configs[1] ("c2": batch 256 x seq 512,
@@ -54,7 +58,14 @@ def parse_args():
                    help="bracket the HBM-resident timed region with cudaProfilerStart/Stop (for ncu --profile-from-start off)")
     p.add_argument("--skip-e2e", action="store_true", help="(profiling only) skip the host-buffer timed region")
     p.add_argument("--no-extra", action="store_true", help="skip the extra_configs block (C1/C3/C4 per-GPU shapes, 3 steps each)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the outputs of the last timed step as DIR/<name>.npy (GPU train() arm only)")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be >= 1")
+    if args.dump_outputs is not None and (args.impl == "reference" or CONFIGS[args.config].get("stream")):
+        p.error("--dump-outputs applies to the GPU train() arm, not to --impl reference or the stream config")
+    return args
 
 
 def resolve_config(args):
@@ -230,6 +241,11 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         time.sleep(0.25)
         self.proc.terminate()
+        try:                                         # reaped here, so that no sampler outlives the run
+            self.proc.wait(timeout=5)
+        except subprocess.TimeoutExpired:
+            self.proc.kill()
+            self.proc.wait()
         sm = sorted(int(r[0]) for r in self.rows if r and r[0].isdigit())
         mx = [int(r[1]) for r in self.rows if len(r) > 1 and r[1].isdigit()]
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
@@ -350,9 +366,35 @@ def measure_prep(opt, rollouts, repeats=2):
     return batch, ms, kern
 
 
-def measure_config(cfg, args, world, rank, dev, steps, warmup, with_e2e):
+DUMP_MAX_ELEMENTS = 1 << 21       # larger arrays are dumped as a fixed seeded sample of this many elements
+DUMP_MAX_BYTES = 64 << 20
+
+
+def step_outputs(opt, result):
+    """What one train() call hands its caller, as host arrays named for --dump-outputs: the loss terms, per-head entropies and
+    grad norms it returns, and the policy parameters it updates in place.  An array of more than DUMP_MAX_ELEMENTS elements
+    (recurrent weights of cells far wider than the BASELINE ones) is replaced by its flattened values at the sorted positions
+    np.random.default_rng(0).choice(n, DUMP_MAX_ELEMENTS, replace=False), the same in every run and every build."""
+    import numpy as np
+    losses, entropies, norms = result
+    named = dict(losses)
+    named.update(("entropy." + k, v) for k, v in entropies.items())
+    named.update(("grad_norm." + k, v) for k, v in norms.items())
+    named.update(("param." + k, v) for k, v in opt.policy_base.state_dict().items())
+    out = {}
+    for name, v in named.items():
+        a = v.detach().cpu().numpy()
+        if a.size > DUMP_MAX_ELEMENTS:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMENTS, replace=False))]
+        out[name] = a
+    assert sum(a.nbytes for a in out.values()) <= DUMP_MAX_BYTES
+    return out
+
+
+def measure_config(cfg, args, world, rank, dev, steps, warmup, with_e2e, dump=False):
     """One BASELINE configuration on this rank's GPU: prep, `steps` timed train() calls (inputs resident in HBM), optional
-    end-to-end loops from pinned host memory.  Returns a dict of raw measurements (rank-local except the max-over-ranks ms)."""
+    end-to-end loops from pinned host memory.  Returns a dict of raw measurements (rank-local except the max-over-ranks ms);
+    with ``dump``, ``outputs`` holds ``step_outputs`` of the last timed step."""
     import torch
     import torch.distributed as dist
     from dotaclient_b200 import ops
@@ -385,10 +427,10 @@ def measure_config(cfg, args, world, rank, dev, steps, warmup, with_e2e):
         barrier()
         return float(ms.item())
 
-    enqueue = []
+    enqueue, last = [], [None]
 
     def step_dev():
-        opt.train(batch_dev)
+        last[0] = opt.train(batch_dev)
         enqueue.append(opt.host_enqueue_s)
 
     for _ in range(max(3, warmup)):
@@ -401,6 +443,7 @@ def measure_config(cfg, args, world, rank, dev, steps, warmup, with_e2e):
         torch.cuda.profiler.stop()
     enq = 1e3 * sum(enqueue[-steps:]) / steps
     graphed = any(isinstance(v, tuple) for v in opt._graphs.values())
+    outputs = step_outputs(opt, last[0]) if dump else None      # before the steps below move the parameters on
     # (2) the same steps launch by launch with CUDA events around every C-ABI call: the per-kernel table of the roofline
     ops.PROFILE.reset(enabled=True)
     step_dev()                                  # untimed: the launch-by-launch path re-grows its allocator pool after the capture
@@ -413,7 +456,7 @@ def measure_config(cfg, args, world, rank, dev, steps, warmup, with_e2e):
     out = {"ms_per_step": ms_total / steps, "ms_per_step_launch_by_launch": ms_eager / steps, "cuda_graph": graphed,
            "prep_ms": prep_ms, "prep_kernels": prep_kern, "kernels": prof, "kernel_bytes": prof_bytes,
            "launches": launches, "host_enqueue_ms": enq, "host_enqueue_ms_launch_by_launch": 1e3 * sum(enqueue[-steps:]) / steps,
-           "h2d_bytes": batch_dev.nbytes()}
+           "h2d_bytes": batch_dev.nbytes(), "outputs": outputs}
     log("[%s] timed region (HBM-resident): %.2f ms/step" % (cfg["name"], out["ms_per_step"]))
     if with_e2e:
         batch_host = batch_dev.pin_memory()
@@ -629,7 +672,8 @@ def main():
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    meas = measure_config(cfg, args, world, rank, dev, args.steps, args.warmup, with_e2e=not args.skip_e2e)
+    meas = measure_config(cfg, args, world, rank, dev, args.steps, args.warmup, with_e2e=not args.skip_e2e,
+                          dump=args.dump_outputs is not None and rank == 0)
     clocks = sampler.stop() if rank == 0 else None
 
     # the other single-GPU-sized BASELINE configurations (per-GPU shapes of C1 / C3 / C4), 3 timed steps each: driver-timed
@@ -712,6 +756,12 @@ def main():
         v, cores, sample, b_sample = cpu_reference_steps_per_sec(cfg, budget_s=20.0)
         line["cpu_baseline"] = {"value": v, "unit": "steps/s", "cores": cores, "kind": "port", "sample": sample,
                                 "sample_batch": b_sample, "scale_factor": b_sample / float(B)}
+    if args.dump_outputs is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in meas["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+        log("wrote %d arrays of the last timed step to %s" % (len(meas["outputs"]), args.dump_outputs))
     emit(line)
     finish_process(world)
 

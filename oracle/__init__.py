@@ -11,11 +11,10 @@ Parity status: the reference (TimZaman/dotaclient @ 8615b90) ships NO tests,
 golden vectors or fixtures for this path (SURVEY.md section 4), so the oracle is
 pinned against *outputs of the reference itself run in the build container*
 (``oracle/reference_shim.py`` imports ``/root/reference`` in place; the script
-``tests/golden/make_golden.py`` records its outputs as committed fixtures, and
-``tests/test_oracle_vs_reference.py`` re-checks bit-equality whenever
-``/root/reference`` is present).  The arithmetic itself lives in third-party,
-un-vendored dependencies of the reference (torch==1.0.0, scipy==1.2.0 --
-``docker/Dockerfile:17-19``); the versions available here are torch 2.11 and
+``tests/golden/make_golden.py`` records its outputs as committed fixtures, which
+``tests/test_oracle.py`` checks the oracle against bit for bit).  The arithmetic
+itself lives in third-party, un-vendored dependencies of the reference
+(torch==1.0.0, scipy==1.2.0 -- ``docker/Dockerfile:17-19``); the versions available here are torch 2.11 and
 scipy 1.18, which is the only executable truth (drift documented in DESIGN.md).
 
 Modules

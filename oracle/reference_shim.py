@@ -4,9 +4,8 @@ TEST INFRASTRUCTURE ONLY.  Works only where ``/root/reference`` exists (the buil
 container); the GPU box never has it, so nothing in ``-m gpu`` tests, ``smoke()``
 or ``bench.py`` may call this.  It is used by
 
-* ``tests/golden/make_golden.py``  -- records reference outputs as fixtures
-* ``tests/test_oracle_vs_reference.py`` -- pins the restatement in ``oracle/``
-  bit-for-bit against the reference (skipped when /root/reference is absent)
+* ``tests/golden/make_golden.py``  -- records reference outputs as the fixtures
+  that ``tests/test_oracle.py`` pins the restatement in ``oracle/`` against
 
 The reference's ``optimizer.py`` imports four packages that are not installed
 here (``optimizer.py:16-17,19,25``); they are irrelevant to the arithmetic, so we

@@ -58,8 +58,10 @@ def test_version_and_argument_errors_without_gpu(lib):
 
 def test_sass_is_sm100a_only():
     import subprocess
+    from dotaclient_b200 import build
     so = os.path.join(ROOT, "dotaclient_b200", "libdotaclient_b200.so")
-    out = subprocess.run(["cuobjdump", "-lelf", so], capture_output=True, text=True).stdout
+    cuobjdump = os.path.join(os.path.dirname(build._nvcc()), "cuobjdump")          # the toolkit that built the library
+    out = subprocess.run([cuobjdump, "-lelf", so], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_(\d+a?)", out))
     assert archs == {"100a"}, archs
 

@@ -293,6 +293,31 @@ def test_bench_config_is_identical_in_both_arms_and_names_the_workload():
     assert bench.algorithmic_rnn_bytes(cfg) == 12.0 * 256 * 512 * 5 * 128            # SURVEY.md 8(d), LSTM: G + 1 = 5
 
 
+def test_bench_step_outputs_names_dtypes_and_sampling():
+    """--dump-outputs: one float array per returned scalar and per parameter, a wide cell's recurrent weights sampled at the
+    same positions on every call, the whole dump under 64 MB even at the widest cell the recurrence accepts (H = 2048)."""
+    import types
+    import bench
+    from dotaclient_b200.policy import Policy
+    keys = ("enum", "x", "y", "target_unit", "ability")
+    result = ({k: torch.tensor(float(i)) for i, k in enumerate(("loss", "policy_loss", "entropy_loss", "value_loss"))},
+              {k: torch.tensor(0.5) for k in keys}, {"unclipped": torch.tensor(2.0), "clipped": torch.tensor(1.0)})
+    torch.manual_seed(7)
+    small = types.SimpleNamespace(policy_base=Policy(hidden_size=128, cell="lstm"))
+    out = bench.step_outputs(small, result)
+    assert len(out) == 4 + 5 + 2 + 34 and float(out["value_loss"]) == 3.0 and float(out["grad_norm.clipped"]) == 1.0
+    assert all(a.dtype in (np.float32, np.float64) for a in out.values())
+    for k, v in small.policy_base.state_dict().items():
+        assert np.array_equal(out["param." + k], v.numpy()), k                      # BASELINE widths: every element
+    wide = types.SimpleNamespace(policy_base=Policy(hidden_size=2048, cell="lstm"))
+    a, b = bench.step_outputs(wide, result), bench.step_outputs(wide, result)
+    w = wide.policy_base.rnn.weight_hh_l0.detach().reshape(-1).numpy()
+    idx = np.sort(np.random.default_rng(0).choice(w.size, bench.DUMP_MAX_ELEMENTS, replace=False))        # the documented positions
+    assert np.array_equal(a["param.rnn.weight_hh_l0"], w[idx])
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+    assert sum(v.nbytes for v in a.values()) <= 64 << 20
+
+
 def test_kernel_traffic_json_matches_the_committed_ncu_csv(tmp_path):
     """profiles/kernel_traffic.json (read by bench.py for roofline.traffic) is derived from profiles/r2_ncu_traffic_c2.csv."""
     import csv

@@ -1,15 +1,13 @@
-"""CPU tests: the oracle against the reference's recorded outputs (tests/golden) and, where the
-reference tree is present (build container), against the reference itself bit-for-bit."""
+"""CPU tests: the oracle against the reference's recorded outputs (tests/golden, written by tests/golden/make_golden.py)."""
 import copy
 import ctypes
+import hashlib
 import os
 import subprocess
 
 import numpy as np
-import pytest
 import torch
 
-from oracle import reference_shim
 from oracle import ref_optimizer as RO
 from oracle.ref_policy import RefPolicy, masked_softmax, sample_index
 from dotaclient_b200.synthetic import make_rollout
@@ -106,28 +104,37 @@ def test_oracle_reproduces_reference_golden(golden):
     np.testing.assert_array_equal(sd["rnn.bias_hh_l0"].numpy(), golden["final_rnn_bias_hh"])
 
 
-@pytest.mark.skipif(not reference_shim.available(), reason="reference tree not present (GPU box)")
+def _load_golden(name):
+    return np.load(os.path.join(ROOT, "tests", "golden", name))
+
+
+def _assert_state_dict_matches(sd, golden, prefix):
+    """Bit for bit against a state dict recorded by make_golden.record_state_dict: the sampled elements first (a mismatch
+    shows its size), then the SHA-256 of every whole tensor."""
+    assert sorted(sd) == sorted(k[len(prefix) + 4:] for k in golden.files if k.startswith(prefix + "val."))
+    for name, t in sd.items():
+        flat = t.detach().reshape(-1).numpy()
+        np.testing.assert_array_equal(flat[golden[prefix + "idx." + name]], golden[prefix + "val." + name], err_msg=name)
+        assert hashlib.sha256(flat.tobytes()).hexdigest() == str(golden[prefix + "sha256." + name]), name
+
+
 def test_oracle_bit_identical_to_reference_live():
-    """Restatement vs the reference imported in place, ragged rollout, 2 epochs."""
+    """Restatement vs the reference's own run (recorded in tests/golden/reference_ragged_seq8.npz), ragged rollout, 2 epochs."""
+    golden = _load_golden("reference_ragged_seq8.npz")
     torch.set_num_threads(1)
-    ref = reference_shim.make_reference_optimizer(seq_len=8)
     mine = _oracle(8)
-    data = make_rollout(29, 5)
-    with torch.no_grad():
-        xr = ref.experiences_from_rollout(copy.deepcopy(data))
-    xm = mine.experiences_from_rollout(copy.deepcopy(data))
-    assert len(xr) == len(xm) == 4
-    for a, b in zip(xr, xm):
-        assert torch.equal(a.advantages, b.advantages) and torch.equal(a.returns, b.returns)
-        assert torch.equal(a.hidden, b.hidden)
-    for _ in range(2):
-        lr_, er_, gr_ = ref.train(xr)
+    xm = mine.experiences_from_rollout(copy.deepcopy(make_rollout(29, 5)))
+    assert len(xm) == len(golden["advantages"]) == 4
+    np.testing.assert_array_equal(np.stack([s.advantages.numpy() for s in xm]), golden["advantages"])
+    np.testing.assert_array_equal(np.stack([s.returns.numpy() for s in xm]), golden["returns"])
+    np.testing.assert_array_equal(np.stack([s.hidden.numpy() for s in xm]), golden["hidden"])
+    for ep in range(2):
         lm_, em_, gm_ = mine.train(xm)
-        assert all(torch.equal(lr_[k], lm_[k]) for k in lr_)
-        assert all(torch.equal(er_[k], em_[k]) for k in er_)
-        assert torch.equal(gr_["unclipped"], gm_["unclipped"]) and torch.equal(gr_["clipped"], gm_["clipped"])
-    for (n, p), (_, q) in zip(ref.policy_base.state_dict().items(), mine.policy_base.state_dict().items()):
-        assert torch.equal(p, q), n
+        np.testing.assert_array_equal(np.stack([lm_[k].detach().numpy() for k in ("loss", "policy_loss", "entropy_loss",
+                                                                                   "value_loss")]), golden["losses"][ep])
+        np.testing.assert_array_equal(np.stack([em_[k].detach().numpy() for k in HEADS]), golden["entropies"][ep])
+        np.testing.assert_array_equal(np.stack([gm_[k].detach().numpy() for k in ("unclipped", "clipped")]), golden["grad_norms"][ep])
+    _assert_state_dict_matches(mine.policy_base.state_dict(), golden, "final_")
 
 
 def test_oracle_lstm_and_width_variants_run():
@@ -165,52 +172,24 @@ def test_sample_index_function():
 
 
 # ------------------------------------------------------------------------------------------------ N-rank oracle
-def _reference_rank_worker(rank, world, port, out_dir):
-    """Runs the UNMODIFIED reference distributed.py + optimizer.train under gloo (SURVEY.md 0.4: prep through policy_base)."""
-    import torch.distributed as dist
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
-    torch.set_num_threads(1)
-    dist.init_process_group("gloo", rank=rank, world_size=world)
-    O, P, D = reference_shim.load()
-    opt = reference_shim.make_reference_optimizer(seq_len=8)
-    with torch.no_grad():
-        xs = opt.experiences_from_rollout(make_rollout(24, 300 + rank))
-    opt.policy = D.DistributedDataParallelSparseParamCPU(opt.policy_base)
-    opt.optimizer = torch.optim.Adam(opt.policy.parameters(), lr=5e-5)
-    recs = []
-    for _ in range(2):
-        l, e, g = opt.train(xs)
-        recs.append(([float(l[k]) for k in ("loss", "policy_loss", "entropy_loss", "value_loss")],
-                     float(g["unclipped"]), float(g["clipped"])))
-    torch.save({"recs": recs, "sd": opt.policy_base.state_dict()}, os.path.join(out_dir, "ref_rank%d.pt" % rank))
-    dist.destroy_process_group()
-
-
-@pytest.mark.skipif(not reference_shim.available(), reason="reference tree not present (GPU box)")
-def test_nrank_oracle_matches_reference_under_gloo(tmp_path):
-    """oracle/ref_distributed.py (one-process emulation) == 2 gloo processes running the reference's wrapper."""
-    import socket
-    import torch.multiprocessing as mp
+def test_nrank_oracle_matches_reference_under_gloo():
+    """oracle/ref_distributed.py (one-process emulation) == 2 gloo processes running the reference's wrapper (recorded in
+    tests/golden/reference_gloo_world2.npz).  The emulation performs the float32 sums of gloo's two-rank all-reduce, so
+    the final weights of both ranks match the recording bit for bit."""
     from oracle import ref_distributed
-    s = socket.socket()
-    s.bind(("127.0.0.1", 0))
-    port = s.getsockname()[1]
-    s.close()
-    mp.spawn(_reference_rank_worker, args=(2, port, str(tmp_path)), nprocs=2, join=True)
+    golden = _load_golden("reference_gloo_world2.npz")
     torch.set_num_threads(1)
     opts = [_oracle(8) for _ in range(2)]
     shards = [opts[r].experiences_from_rollout(make_rollout(24, 300 + r)) for r in range(2)]
     mine = [ref_distributed.train_ranks(opts, shards) for _ in range(2)]
     for r in range(2):
-        ref = torch.load(os.path.join(str(tmp_path), "ref_rank%d.pt" % r))
         for ep in range(2):
             l, e, g = mine[ep][r]
             got = [float(l[k]) for k in ("loss", "policy_loss", "entropy_loss", "value_loss")]
-            np.testing.assert_array_equal(np.array(got), np.array(ref["recs"][ep][0]))
-            np.testing.assert_allclose(float(g["unclipped"]), ref["recs"][ep][1], rtol=1e-6)
-            np.testing.assert_allclose(float(g["clipped"]), ref["recs"][ep][2], rtol=1e-6)
-        for k, v in opts[r].policy_base.state_dict().items():
-            torch.testing.assert_close(v, ref["sd"][k], rtol=0, atol=1e-7, msg=lambda m: k + m)
+            np.testing.assert_array_equal(np.array(got), golden["rank%d_losses" % r][ep])
+            np.testing.assert_allclose(float(g["unclipped"]), golden["rank%d_grad_norms" % r][ep][0], rtol=1e-6)
+            np.testing.assert_allclose(float(g["clipped"]), golden["rank%d_grad_norms" % r][ep][1], rtol=1e-6)
+        _assert_state_dict_matches(opts[r].policy_base.state_dict(), golden, "rank%d_final_" % r)
 
 
 def test_target_unit_head_is_linear_in_the_unit_embedding():
