@@ -31,12 +31,14 @@ SIGNATURES = {
     "dc_gemm_wgrad_tf32x3_blocked": (_i32, [_vp, _i32, _i64, _i64, _vp, _i32, _i64, _i32, _i32, _vp, _i32, _vp, _i32, _vp,
                                             _vp]),
     "dc_unit_basic_fwd": (_i32, [_vp, _vp, _vp, _vp, _i64, _vp]),
+    "dc_unit_basic_fwd_mask": (_i32, [_vp, _vp, _vp, _vp, _vp, _i64, _vp]),
     "dc_unit_basic_bwd_workspace_bytes": (_sz, []),
     "dc_env_fwd": (_i32, [_vp, _vp, _vp, _vp, _i32, _i64, _vp]),
     "dc_env_bwd_workspace_bytes": (_sz, []),
     "dc_env_bwd": (_i32, [_vp, _vp, _i32, _vp, _vp, _vp, _i64, _vp, _vp]),
     "dc_unit_wgrad_routed": (_i32, [_vp, _vp, _i32, _vp, _vp, _i64, _i32, _vp, _vp, _vp, _vp]),
     "dc_unit_dgrad_fused": (_i32, [_vp, _vp, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _i32, _vp, _vp]),
+    "dc_unit_dgrad_fused_mask": (_i32, [_vp, _vp, _i32, _vp, _vp, _i32, _vp, _vp, _vp, _vp, _i64, _i32, _vp, _vp, _i32, _vp, _vp]),
     "dc_gemm_unit_max": (_i32, [_vp, _vp, _vp, _vp, _vp, _i32, _vp, _i64, _i32, _vp]),
     "dc_target_unit_q_fwd": (_i32, [_vp, _i32, _c.c_void_p * 6, _vp, _i64, _vp]),
     "dc_target_unit_q_bwd": (_i32, [_vp, _c.c_void_p * 6, _vp, _i32, _i64, _vp]),

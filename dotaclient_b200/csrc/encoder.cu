@@ -5,7 +5,8 @@
 //
 //   env_fwd / env_bwd   relu(env W_e^T + b_e), 3 -> 128, written into / read from columns [0,128) of the concatenated
 //                       [N, 896] pre-rnn input row (no torch.cat), policy.py:55,97
-//   unit_basic_fwd      relu(units W_b^T + b_b)            [R,12] -> [R,128]     (K = 12: not a tensor-core shape)
+//   unit_basic_fwd      relu(units W_b^T + b_b)            [R,12] -> [R,128]     (K = 12: not a tensor-core shape),
+//                       optionally with its ReLU sign bits for the data-gradient kernel
 //   unit_basic reduce   fixed-order sum of the dW_b / db_b partials of the fused data-gradient kernel (gemm_tf32x3.cu)
 //   target_unit_q_fwd   logits[n,u] = <att[n] W_g, basic[n,u]> + <att[n], b_g>: the head WITHOUT the [N,40,128] embedding
 //   target_unit_q_bwd   s_g[n] = sum_u dlogits[n,u] basic_g[n,u] (-> d_att and the head's share of dW_g as token-level GEMMs)
@@ -26,10 +27,15 @@ constexpr int kThreadsE = kWarps * 32;
 constexpr int kMaxUnits = 40;
 
 // ---- relu(units W_b^T + b_b) -------------------------------------------------------------------
+// mask (optional): the ReLU sign bits for the data-gradient kernel, uint32 [ceil(R/32)][128] with bit i of word [b][j] =
+// basic[32b + i][j] > 0 (bits of rows >= R are 0).  A warp iteration owns 32 rows starting at a multiple of 32 and lane l owns
+// channels 4l..4l+3, so a lane collects one bit per row in four registers and stores one 16-byte word per iteration (512 coalesced
+// bytes per warp).  The bit is taken from the value written to `basic`, so the backward sees exactly the forward's mask.
 __global__ void __launch_bounds__(kThreadsE) unit_basic_fwd_kernel(const float *__restrict__ units,
                                                                    const float *__restrict__ w_b,
                                                                    const float *__restrict__ b_b,
-                                                                   float *__restrict__ basic, int64_t R) {
+                                                                   float *__restrict__ basic, uint32_t *__restrict__ mask,
+                                                                   int64_t R) {
     __shared__ float s_u[kWarps][32][kIn];                        // 32 rows of raw features per warp per iteration
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     // weights as channel PAIRS for the packed fp32x2 FMA (FFMA2): w2[p][k] = (W_b[4l+2p][k], W_b[4l+2p+1][k])
@@ -47,6 +53,7 @@ __global__ void __launch_bounds__(kThreadsE) unit_basic_fwd_kernel(const float *
         float *su = &s_u[warp][0][0];
         for (int i = lane; i < nrows * kIn; i += 32) su[i] = units[base * kIn + i];
         __syncwarp();
+        uint4 bits = make_uint4(0u, 0u, 0u, 0u);
         for (int r = 0; r < nrows; ++r) {
             float2 a0 = b2[0], a1 = b2[1];
 #pragma unroll
@@ -56,9 +63,12 @@ __global__ void __launch_bounds__(kThreadsE) unit_basic_fwd_kernel(const float *
                 a0 = __ffma2_rn(uu, w2[0][k], a0);
                 a1 = __ffma2_rn(uu, w2[1][k], a1);
             }
-            *reinterpret_cast<float4 *>(basic + (base + r) * kC + lane * 4) =
-                make_float4(fmaxf(a0.x, 0.f), fmaxf(a0.y, 0.f), fmaxf(a1.x, 0.f), fmaxf(a1.y, 0.f));
+            const float4 o = make_float4(fmaxf(a0.x, 0.f), fmaxf(a0.y, 0.f), fmaxf(a1.x, 0.f), fmaxf(a1.y, 0.f));
+            *reinterpret_cast<float4 *>(basic + (base + r) * kC + lane * 4) = o;
+            bits.x |= (uint32_t)(o.x > 0.f) << r; bits.y |= (uint32_t)(o.y > 0.f) << r;
+            bits.z |= (uint32_t)(o.z > 0.f) << r; bits.w |= (uint32_t)(o.w > 0.f) << r;
         }
+        if (mask != nullptr) *reinterpret_cast<uint4 *>(mask + (base >> 5) * kC + lane * 4) = bits;
         __syncwarp();
     }
 }
@@ -323,7 +333,17 @@ extern "C" int dc_unit_basic_fwd(const float *units, const float *w_b, const flo
                                  dc_stream_t stream) {
     DC_REQUIRE(units && w_b && b_b && basic && R > 0, DC_EINVAL, "dc_unit_basic_fwd: bad arguments");
     DC_REQUIRE(((uintptr_t)basic & 15) == 0, DC_EINVAL, "dc_unit_basic_fwd: output must be 16-byte aligned");
-    unit_basic_fwd_kernel<<<grid_rows(0), kThreadsE, 0, dc_cu_stream(stream)>>>(units, w_b, b_b, basic, R);
+    unit_basic_fwd_kernel<<<grid_rows(0), kThreadsE, 0, dc_cu_stream(stream)>>>(units, w_b, b_b, basic, nullptr, R);
+    DC_LAUNCH_OK();
+    return DC_OK;
+}
+
+extern "C" int dc_unit_basic_fwd_mask(const float *units, const float *w_b, const float *b_b, float *basic, uint32_t *mask,
+                                      int64_t R, dc_stream_t stream) {
+    DC_REQUIRE(units && w_b && b_b && basic && mask && R > 0, DC_EINVAL, "dc_unit_basic_fwd_mask: bad arguments");
+    DC_REQUIRE(((uintptr_t)basic & 15) == 0 && ((uintptr_t)mask & 15) == 0, DC_EINVAL,
+               "dc_unit_basic_fwd_mask: basic and mask must be 16-byte aligned");
+    unit_basic_fwd_kernel<<<grid_rows(0), kThreadsE, 0, dc_cu_stream(stream)>>>(units, w_b, b_b, basic, mask, R);
     DC_LAUNCH_OK();
     return DC_OK;
 }

@@ -62,8 +62,8 @@ def _wgrad_workspace(No, Ni, device):
 # dense [N, 40, 128] tensor at all:
 #   dW_g  = R^T basic_g  (dc_unit_wgrad_routed: R generated in the A producer)  +  att^T s_g   (one token-level GEMM for all groups,
 #           s_g = sum_u dlogits_u basic_u from dc_target_unit_q_bwd; its bias block gives the head's share of db_g)
-#   dW_b += (relu'(.) (R + dlogits x att) W_g)^T units   (dc_unit_dgrad_fused: d_emb generated in the producers, the ReLU mask
-#           recomputed and dW_b reduced in the epilogue) -- d_basic never exists either.
+#   dW_b += (relu'(.) (R + dlogits x att) W_g)^T units   (dc_unit_dgrad_fused_mask: d_emb generated in the producers, the ReLU mask
+#           read as the bits the forward stored next to `basic`, dW_b reduced in the epilogue) -- d_basic never exists either.
 
 
 def _ptr(t, float_offset=0):
@@ -83,7 +83,7 @@ class UnitEncoder(torch.autograd.Function):
     """
 
     @staticmethod
-    def forward(ctx, link, env, w_e, b_e, w_b, b_b, *rest):
+    def forward(ctx, link, keep_mask, env, w_e, b_e, w_b, b_b, *rest):
         units, weights, biases = rest[:6], rest[6:12], rest[12:18]
         ctx.link = link
         _need_cuda(env, w_b, *units)
@@ -106,14 +106,21 @@ class UnitEncoder(torch.autograd.Function):
         wait_h2d(env2)
         with PROFILE.span("env_fwd", 1, 4 * N * (3 + C)):
             _lib.check(lib.dc_env_fwd(env2.data_ptr(), w_e.data_ptr(), b_e.data_ptr(), xcat.data_ptr(), XCAT, N, st), "dc_env_fwd")
-        basics = []
+        basics, masks = [], []
         for g, n_u in enumerate(UNITS):
             R = N * n_u
             basic = torch.empty((R, C), dtype=torch.float32, device=dev)
             wait_h2d(units[g])                       # this group's observations may still be in flight over PCIe
-            with PROFILE.span("unit_basic_fwd", 1, 4 * R * (12 + C)):
-                _lib.check(lib.dc_unit_basic_fwd(units[g].data_ptr(), w_b.data_ptr(), b_b.data_ptr(), basic.data_ptr(), R, st),
-                           "dc_unit_basic_fwd")
+            if keep_mask:                            # the ReLU sign bits of `basic` for the backward: 1/32 of its bytes
+                mask = torch.empty(((R + 31) // 32, C), dtype=torch.int32, device=dev)
+                with PROFILE.span("unit_basic_fwd", 1, 4 * R * (12 + C) + mask.numel() * 4):
+                    _lib.check(lib.dc_unit_basic_fwd_mask(units[g].data_ptr(), w_b.data_ptr(), b_b.data_ptr(), basic.data_ptr(),
+                                                          mask.data_ptr(), R, st), "dc_unit_basic_fwd_mask")
+                masks.append(mask)
+            else:
+                with PROFILE.span("unit_basic_fwd", 1, 4 * R * (12 + C)):
+                    _lib.check(lib.dc_unit_basic_fwd(units[g].data_ptr(), w_b.data_ptr(), b_b.data_ptr(), basic.data_ptr(), R, st),
+                               "dc_unit_basic_fwd")
             if n_u > 1:                               # embedding GEMM with the max-pool in its epilogue
                 copy = _ptr(xcat, 6 * C) if g == 3 else None
                 with PROFILE.span("gemm_unit_max", 1, 4 * (R * C + C * C + N * C) + N * C):
@@ -128,14 +135,15 @@ class UnitEncoder(torch.autograd.Function):
         link["basics"], link["weights"], link["biases"] = basics, weights, biases
         ctx.N = N
         ctx.lead = lead
-        ctx.save_for_backward(argmax, *units, *basics, *weights, env2, xcat, w_b, b_b)
+        ctx.keep_mask = keep_mask
+        ctx.save_for_backward(argmax, *units, *basics, *weights, env2, xcat, *masks)
         return xcat.view(*lead, XCAT)
 
     @staticmethod
     def backward(ctx, d_xcat):
         saved = ctx.saved_tensors
         argmax, units, basics, weights, env2, xcat = saved[0], saved[1:7], saved[7:13], saved[13:19], saved[19], saved[20]
-        w_b, b_b = saved[21], saved[22]
+        masks = saved[21:27]
         N = ctx.N
         lib = _lib.load()
         st = _lib.stream_ptr()
@@ -150,8 +158,10 @@ class UnitEncoder(torch.autograd.Function):
         dl = att = s_head = None
         if pending is not None:
             dl, att, s_head = pending
-        dw_b = torch.empty((C, 12), dtype=torch.float32, device=dev)
-        db_b = torch.empty(C, dtype=torch.float32, device=dev)
+        dw_b = db_b = None                              # the forward kept the ReLU mask iff w_b / b_b need a gradient
+        if ctx.keep_mask:
+            dw_b = torch.empty((C, 12), dtype=torch.float32, device=dev)
+            db_b = torch.empty(C, dtype=torch.float32, device=dev)
         dw_all = torch.zeros((6, C, C), dtype=torch.float32, device=dev)     # zeros: the enemy-tower layer has no max-pool path
         db_all = torch.zeros((6, C), dtype=torch.float32, device=dev)
         ws_w = _wgrad_workspace(C, C, dev)
@@ -170,13 +180,16 @@ class UnitEncoder(torch.autograd.Function):
                 with PROFILE.span("gemm_wgrad", 2, 4 * (2 * R * C + C * C)):
                     _lib.check(lib.dc_gemm_wgrad_tf32x3(dx, XCAT, basics[g].data_ptr(), C, R, C, C, dw_all[g].data_ptr(), C,
                                                         db_all[g].data_ptr(), 0, ws_w.data_ptr(), st), "dc_gemm_wgrad_tf32x3")
+            if not ctx.keep_mask:
+                continue
             wt = weights[g].t().contiguous()
-            with PROFILE.span("unit_dgrad_fused", 2, N * (4 * C + C) * (1 if routed else 0) + 4 * R * 12 + (4 * N * (C + n_u) if dl is not None else 0)):
-                _lib.check(lib.dc_unit_dgrad_fused(dx, dx2, XCAT, argmax[g].data_ptr() if (routed and n_u > 1) else None,
-                                                   None if dl is None else _ptr(dl, off), MAX_UNITS, None if att is None else att.data_ptr(),
-                                                   wt.data_ptr(), units[g].data_ptr(), w_b.data_ptr(), b_b.data_ptr(), N, n_u,
-                                                   dw_b.data_ptr(), db_b.data_ptr(), 1 if g > 0 else 0, ws_b.data_ptr(), st),
-                           "dc_unit_dgrad_fused")
+            with PROFILE.span("unit_dgrad_fused", 2, N * (4 * C + C) * (1 if routed else 0) + 4 * R * 12 + masks[g].numel() * 4 +
+                              (4 * N * (C + n_u) if dl is not None else 0)):
+                _lib.check(lib.dc_unit_dgrad_fused_mask(dx, dx2, XCAT, argmax[g].data_ptr() if (routed and n_u > 1) else None,
+                                                        None if dl is None else _ptr(dl, off), MAX_UNITS,
+                                                        None if att is None else att.data_ptr(), wt.data_ptr(), units[g].data_ptr(),
+                                                        masks[g].data_ptr(), N, n_u, dw_b.data_ptr(), db_b.data_ptr(), 1 if g > 0 else 0,
+                                                        ws_b.data_ptr(), st), "dc_unit_dgrad_fused_mask")
         if dl is not None:
             # the head's share of every dW_g and db_g in ONE token-level product: att^T [s_0 | ... | s_5 | sum_u dlogits]
             dw_head = torch.empty((C, QW), dtype=torch.float32, device=dev)
@@ -186,7 +199,7 @@ class UnitEncoder(torch.autograd.Function):
             dw_all += dw_head[:, :6 * C].reshape(C, 6, C).permute(1, 0, 2)
             db_all += dw_head[:, 6 * C:6 * C + 6].t()
         dws, dbs = list(dw_all.unbind(0)), list(db_all.unbind(0))
-        return (None, None, dw_e, db_e, dw_b, db_b) + (None,) * 6 + tuple(dws) + tuple(dbs)
+        return (None, None, None, dw_e, db_e, dw_b, db_b) + (None,) * 6 + tuple(dws) + tuple(dbs)
 
 
 QW = 7 * C     # width of the head's token-level operands: six groups x 128 channels + one block carrying the six bias dots
@@ -238,7 +251,8 @@ class TargetUnit(torch.autograd.Function):
 def unit_encoder(env, w_e, b_e, w_b, b_b, units, weights, biases):
     """-> (``link``: the handle ``target_unit`` needs, pre-rnn input ``[..., 896]``)."""
     link = {}
-    xcat = UnitEncoder.apply(link, env, w_e, b_e, w_b, b_b, *units, *weights, *biases)
+    keep_mask = torch.is_grad_enabled() and (w_b.requires_grad or b_b.requires_grad)
+    xcat = UnitEncoder.apply(link, keep_mask, env, w_e, b_e, w_b, b_b, *units, *weights, *biases)
     return link, xcat
 
 

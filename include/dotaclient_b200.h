@@ -127,6 +127,10 @@ int dc_gemm_wgrad_tf32x3_blocked(const float *dY, int ldy, int64_t y_rows_per_bl
  */
 int dc_unit_basic_fwd(const float *units, const float *w_b, const float *b_b, float *basic, int64_t R,
                       dc_stream_t stream);
+/* The same, also writing the ReLU sign bits of `basic` for dc_unit_dgrad_fused_mask: mask = uint32 [ceil(R/32), 128], bit i of
+ * word [b][j] = basic[32b + i][j] > 0, bits of rows >= R are 0.  basic and mask 16-byte aligned. */
+int dc_unit_basic_fwd_mask(const float *units, const float *w_b, const float *b_b, float *basic, uint32_t *mask, int64_t R,
+                           dc_stream_t stream);
 size_t dc_unit_basic_bwd_workspace_bytes(void);   /* partial sums of dW_b / db_b: the workspace of dc_unit_dgrad_fused */
 /* Environment encoder (policy.py:55,97): out[n*ld_out + c] = relu(env[n,:3] . W_e[c,:] + b_e[c]), c < 128 -- written into
  * columns [0,128) of the concatenated pre-rnn input row (ld_out = 896), so the reference's torch.cat (policy.py:129-136)
@@ -166,6 +170,12 @@ int dc_unit_dgrad_fused(const float *d_xmax, const float *d_xmax2, int ld_dx, co
                         int ld_dl, const float *att, const float *w_t, const float *units, const float *w_b,
                         const float *b_b, int64_t n_tokens, int n_units, float *dw_b, float *db_b, int accumulate,
                         void *workspace, dc_stream_t stream);
+/* dc_unit_dgrad_fused with the ReLU mask read from the forward pass (dc_unit_basic_fwd_mask of the same rows, 16-byte aligned)
+ * instead of recomputed from w_b, b_b: the same results, bit for bit. */
+int dc_unit_dgrad_fused_mask(const float *d_xmax, const float *d_xmax2, int ld_dx, const uint8_t *argmax, const float *dlogits,
+                             int ld_dl, const float *att, const float *w_t, const float *units, const uint32_t *mask,
+                             int64_t n_tokens, int n_units, float *dw_b, float *db_b, int accumulate, void *workspace,
+                             dc_stream_t stream);
 int dc_target_unit_fwd(const float *att, const float *ue, float *logits, int64_t N, dc_stream_t stream);
 int dc_target_unit_bwd(const float *dlogits, const float *att, const float *ue, float *d_att, float *d_ue,
                        int64_t N, dc_stream_t stream);
